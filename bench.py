@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Issue_Embeddings encoder hot path (BASELINE.json: issues/sec to 2400-d @ seq_len 512 batch 256).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of 256 synthetic issues x 512 tokens (BASELINE.json configs[1]
 shape; reference-deployed R4 encoder: L=4, E=800, H=2400, V=60000, random-init seed 1234): token ids -> per-token
@@ -38,6 +38,16 @@ same measurement with one batch per launch.
                  no network -- see DESIGN.md); each step is a bounded sample (>= 32 issues) of the same workload.
 * `extra`      : fp32-accurate mode (IE_CFG_FP32), the north star's literal 3-layer shape (N3), the device-resident MLP
                  head (configs[4]) and a var-len bulk run checked bit for bit against a single-GPU encode.
+
+`--dump-outputs DIR` writes, after the timed steps, what the timed paths handed back (float32 .npy, 12 MB on one GPU),
+so that two builds can be compared output for output; inputs and weights are seeded, so the same arguments give the
+same inputs:
+* `embeddings.npy`            : the (256, 2400) result of the last timed step of `value` (with G ranks: that step of
+                                every rank, rank-major; above 2048 rows a fixed seeded sample of them)
+* `e2e_embeddings_sample.npy` : rows of the (N, 2400) array `e2e`'s bulk call returned, a fixed seeded sample of at most
+                                1024 rows in ascending row order
+* `reference_embeddings.npy`  : under `--impl reference`, the first 32 rows of the last timed step (how many issues
+                                that arm encodes per step depends on a host-speed probe; the ids of its first rows do not)
 """
 import argparse
 import json
@@ -170,6 +180,28 @@ def cpu_oracle_setup():
     return enc, best[1], best[0], cores
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def sample_rows(a, max_rows, seed=0):
+    """A copy of `a` if it has at most `max_rows` rows, else a fixed seeded sample of them in ascending row order."""
+    import numpy as np
+    if a.shape[0] <= max_rows:
+        return np.array(a)
+    return a[np.sort(np.random.default_rng(seed).choice(a.shape[0], size=max_rows, replace=False))]
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"{total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte dump limit"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def cpu_sample_size(tok_rate, budget_s):
     return int(max(CPU_SAMPLE_MIN, min(B, tok_rate * budget_s / T)))
 
@@ -203,9 +235,11 @@ def run_reference(args):
         R.encode_padded(enc, ids, [T] * sb)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        R.encode_padded(enc, ids, [T] * sb)
+        out = R.encode_padded(enc, ids, [T] * sb)
     dt = time.perf_counter() - t0
     val = sb * args.steps / dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"reference_embeddings": out[:CPU_SAMPLE_MIN]})
     sample = (f"{sb} of the {B} issues of a step (seq_len {T}), torch fp32 nn.LSTM oracle, {threads} threads "
               f"(best of a thread-count probe; {cores} usable cores)")
     print(json.dumps({
@@ -228,7 +262,11 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what they computed as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -324,6 +362,10 @@ def main():
     ms_max, launches, phases, phase_mhz = device_arm(kPerLaunch)   # five batches per launch: the bulk-encode mode
     value = world * B * K / (ms_max * 1e-3)
     single_value = world * B * K / (ms_single * 1e-3)
+    dumps = {}
+    if args.dump_outputs and rank == 0:
+        last = gathered.view(world, K, B, 3 * EMB)[:, K - 1] if world > 1 else out_dev[(K - 1) * B:]
+        dumps["embeddings"] = sample_rows(last.reshape(-1, 3 * EMB).cpu().numpy(), 2048)
 
     # ---- end-to-end arm: HOST token-id lists through the public bulk API -----------------------------------
     # every rank holds the same global list (the reference's per-repo list of numericalised issues), as the API expects
@@ -347,6 +389,8 @@ def main():
     assert tuple(res.shape) == (n_total, 3 * EMB)
     if rank == 0:
         assert isinstance(res, np.ndarray) and np.isfinite(res[::97]).all()
+        if args.dump_outputs:
+            dumps["e2e_embeddings_sample"] = sample_rows(res, 1024)
     t_e2e = torch.tensor([e2e_s], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t_e2e, op=dist.ReduceOp.MAX)
@@ -454,6 +498,8 @@ def main():
             line["cpu_baseline"] = {"value": rate, "unit": "issues/s", "cores": threads, "kind": "port",
                                     "sample": f"{sb} issues x seq_len {T} ({sb}/{B} of a step), torch fp32 nn.LSTM "
                                               f"oracle, {threads} threads of {cores} usable cores, {dt:.1f} s"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

@@ -246,6 +246,23 @@ def test_bench_clock_sampler_summary():
     assert bench.ClockSampler.summarise([])["sm_mhz"] is None
 
 
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: float32 .npy per name, a row sample that is the same on every run, a size cap."""
+    import bench
+    a = np.arange(5000 * 3, dtype=np.float64).reshape(5000, 3)
+    s = bench.sample_rows(a, 1024)
+    assert s.shape == (1024, 3) and np.array_equal(s, bench.sample_rows(a, 1024))
+    assert (np.diff(s[:, 0]) > 0).all() and np.isin(s[:, 0], a[:, 0]).all()
+    small = bench.sample_rows(a[:10], 1024)
+    assert np.array_equal(small, a[:10]) and not np.shares_memory(small, a)
+    bench.dump_outputs(str(tmp_path / "d"), {"embeddings": a[:4], "e2e_embeddings_sample": s})
+    back = np.load(tmp_path / "d" / "embeddings.npy")
+    assert back.dtype == np.float32 and np.array_equal(back, a[:4].astype(np.float32))
+    assert sorted(os.listdir(tmp_path / "d")) == ["e2e_embeddings_sample.npy", "embeddings.npy"]
+    with pytest.raises(AssertionError):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": np.zeros((bench.DUMP_MAX_BYTES // 4 + 1,), np.float32)})
+
+
 def _rot_schedule_model(T, ng, tiles, P, mma, lat, slots=2, pre=0.0):
     """Event model of csrc/lstm_layer.cu's schedule: item n = t*C + g*tiles + j (C = ng*tiles) runs on CTA pair n % P, pairs
     walk their items in increasing n; an item's MMAs start when the pair is free, every item of (t-1, g) has been
