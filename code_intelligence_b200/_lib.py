@@ -48,7 +48,12 @@ PROTOTYPES = {
     "ie_mlp_destroy": (None, [C.c_void_p]),
     "ie_pr_thresholds": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
-    "ie_debug_gemm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+    "ie_knn_create": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                C.POINTER(C.c_void_p)]),
+    "ie_knn_search": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                C.c_int32, C.c_void_p]),
+    "ie_knn_destroy": (None, [C.c_void_p]),
+    "ie_debug_gemm": (C.c_int,[C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                 C.c_void_p, C.c_int32]),
 }
 

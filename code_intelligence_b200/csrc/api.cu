@@ -1,6 +1,7 @@
 // C-ABI layer of libissue_emb_b200.so (declared in include/issue_emb_b200.h): handle management, weight
 // re-layout, workspace, and the launch sequence of the encoder hot path and the MLP head.
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -160,6 +161,28 @@ struct ie_mlp {
   int chunk_dev = 1 << 18;  // rows per pass in device-pointer mode (IE_MLP_CHUNK at create time)
   cudaStream_t own_stream = nullptr;
   std::mutex mu;
+};
+
+struct ie_knn {
+  int device = 0;
+  int num_sms = 148;
+  long long n = 0;
+  int d = 0, k_pad = 0, n_pad = 0;
+  DevBuf index;  // bf16 [n_pad, 2*k_pad]: [hi | lo] of the f32 residual x/|x| - mean; padding rows zero
+  DevBuf bias;   // f32 [n_pad]: b_x = mean . r_x
+  DevBuf omc;    // f64 [n]: 1 - c_x = 1 - (x/|x|) . mean (self-queries)
+  DevBuf mean;   // f64 [k_pad]: mean of the unit vectors
+  // search workspace
+  DevBuf qf, qa, qomc, cand_s, cand_i, dist, ids, err;
+  cudaStream_t own_stream = nullptr;
+  cudaStream_t last_stream = nullptr;
+  cudaEvent_t done_ev = nullptr;  // end of the last call: a call on another stream waits for it (shared workspace)
+  bool has_done = false;
+  std::mutex mu;
+  ~ie_knn() {
+    if (done_ev) cudaEventDestroy(done_ev);
+    if (own_stream) cudaStreamDestroy(own_stream);
+  }
 };
 
 namespace {
@@ -1031,6 +1054,202 @@ int ie_debug_gemm(const float* a, const float* b, const float* bias, int32_t M, 
                   cudaMemcpyDeviceToHost));
   fa.release(); fb.release(); ba.release(); bb.release(); dd.release(); db.release();
   return IE_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// Similar-issue search (knn.cu)
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+constexpr int kKnnMaxDim = 4096;
+constexpr long long kKnnBuildChunk = 1 << 16;  // rows per prep pass (host input is staged through an f32 buffer this big)
+constexpr int kKnnQueryChunk = 2048;           // queries per search launch (bounds the candidate workspace)
+
+int knn_build(ie_knn* h, const float* vectors, bool dev, cudaStream_t s) {
+  const long long n = h->n;
+  const int d = h->d;
+  const long long chunk = std::min(n, kKnnBuildChunk);
+  const long long nblk = ie::knn_colsum_blocks(n);
+  CK(h->index.reserve(static_cast<size_t>(h->n_pad) * 2 * h->k_pad * sizeof(__nv_bfloat16), true));
+  CK(h->bias.reserve(static_cast<size_t>(h->n_pad) * sizeof(float), true));
+  CK(h->omc.reserve(static_cast<size_t>(n) * sizeof(double)));
+  CK(h->mean.reserve(static_cast<size_t>(h->k_pad) * sizeof(double)));
+  CK(h->err.reserve(sizeof(unsigned), true));
+  DevBuf inv, partial, xf;
+  CK(inv.reserve(static_cast<size_t>(chunk) * sizeof(double)));
+  CK(partial.reserve(static_cast<size_t>(nblk) * d * sizeof(double)));
+  if (!dev) CK(xf.reserve(static_cast<size_t>(chunk) * d * sizeof(float)));
+  unsigned* flag = h->err.as<unsigned>();
+  auto rows_at = [&](long long r0, int rows) -> const float* {
+    if (dev) return vectors + r0 * d;
+    if (cudaMemcpyAsync(xf.p, vectors + r0 * d, static_cast<size_t>(rows) * d * sizeof(float), cudaMemcpyHostToDevice,
+                        s) != cudaSuccess)
+      return nullptr;
+    return xf.as<float>();
+  };
+  // pass 1: norms and fixed-order partial column sums of the unit vectors -> mean
+  for (long long r0 = 0; r0 < n; r0 += chunk) {
+    const int rows = static_cast<int>(std::min(chunk, n - r0));
+    const float* x = rows_at(r0, rows);
+    if (x == nullptr) return cuda_fail(cudaGetLastError(), "cudaMemcpyAsync");
+    CK(ie::launch_knn_check_finite(x, d, d, rows, flag, s));
+    CK(ie::launch_knn_inv_norm(x, d, d, rows, inv.as<double>(), s));
+    CK(ie::launch_knn_colsum(x, d, d, rows, inv.as<double>(), partial.as<double>(), r0 / 512, s));
+  }
+  CK(ie::launch_knn_mean(partial.as<double>(), nblk, d, h->k_pad, n, h->mean.as<double>(), s));
+  unsigned bad = 0;
+  CK(cudaMemcpyAsync(&bad, flag, sizeof(unsigned), cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  if (bad) return fail(IE_ERR_INVALID, "vectors contain NaN or infinite values");
+  // pass 2: split-bf16 residuals, b_x and 1 - c_x
+  for (long long r0 = 0; r0 < n; r0 += chunk) {
+    const int rows = static_cast<int>(std::min(chunk, n - r0));
+    const float* x = rows_at(r0, rows);
+    if (x == nullptr) return cuda_fail(cudaGetLastError(), "cudaMemcpyAsync");
+    CK(ie::launch_knn_prep_rows(x, d, d, rows, h->mean.as<double>(), h->k_pad,
+                                h->index.as<__nv_bfloat16>() + r0 * 2 * h->k_pad, h->bias.as<float>() + r0,
+                                h->omc.as<double>() + r0, s));
+  }
+  CK(cudaStreamSynchronize(s));
+  return IE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ie_knn_create(const float* vectors, int64_t n, int32_t d, int32_t device, int32_t flags, void* stream, ie_knn** out) {
+  if (vectors == nullptr || out == nullptr) return fail(IE_ERR_INVALID, "null argument");
+  if (d < 1 || d > kKnnMaxDim) return fail(IE_ERR_INVALID, "d=%d outside [1,%d]", d, kKnnMaxDim);
+  if (n < 1 || n > INT32_MAX - 256) return fail(IE_ERR_INVALID, "n=%lld outside [1,%d]", static_cast<long long>(n), INT32_MAX - 256);
+  int ndev = 0;
+  cudaError_t e = cudaGetDeviceCount(&ndev);
+  if (e != cudaSuccess || ndev == 0)
+    return fail(IE_ERR_CUDA, "no CUDA device available (%s): this library has no CPU fallback", cudaGetErrorString(e));
+  if (device < 0 || device >= ndev) return fail(IE_ERR_INVALID, "device %d not in [0,%d)", device, ndev);
+  CK(cudaSetDevice(device));
+  int major = 0, sms = 0;
+  CK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
+  CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+  if (major != 10) return fail(IE_ERR_CUDA, "device compute capability %d.x is not sm_100 (B200)", major);
+  ie_knn* h = new ie_knn();
+  h->device = device;
+  h->num_sms = sms;
+  h->n = n;
+  h->d = d;
+  h->k_pad = static_cast<int>(round_up(d, 64));
+  h->n_pad = static_cast<int>(round_up(n, 256));
+  e = cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->done_ev, cudaEventDisableTiming);
+  if (e != cudaSuccess) { delete h; return cuda_fail(e, "cudaStreamCreate"); }
+  const bool dev = (flags & IE_FLAG_DEVICE_PTRS) != 0;
+  const int rc = knn_build(h, vectors, dev, dev ? static_cast<cudaStream_t>(stream) : h->own_stream);
+  if (rc != IE_OK) { delete h; return rc; }
+  *out = h;
+  return IE_OK;
+}
+
+int ie_knn_search(ie_knn* h, const float* queries, int64_t row0, int32_t m, int32_t k, float* distances, int64_t* ids,
+                  int32_t flags, void* stream) {
+  if (h == nullptr || distances == nullptr || ids == nullptr) return fail(IE_ERR_INVALID, "null argument");
+  if (m < 1) return fail(IE_ERR_INVALID, "m=%d must be >= 1", m);
+  const bool self = queries == nullptr;
+  const long long cands = self ? h->n - 1 : h->n;
+  if (k < 1 || k > ie::kKnnMaxK) return fail(IE_ERR_INVALID, "k=%d outside [1,%d]", k, ie::kKnnMaxK);
+  if (k > cands) return fail(IE_ERR_INVALID, "k=%d exceeds the %lld candidates of the index", k, cands);
+  if (self && (row0 < 0 || row0 + m > h->n))
+    return fail(IE_ERR_INVALID, "rows [%lld,%lld) outside the index of %lld rows", static_cast<long long>(row0),
+                static_cast<long long>(row0) + m, h->n);
+  const bool dev = (flags & IE_FLAG_DEVICE_PTRS) != 0;
+  const int d = h->d;
+  if (!self && !dev) {
+    const size_t total = static_cast<size_t>(m) * d;
+    for (size_t i = 0; i < total; ++i)
+      if (!std::isfinite(queries[i])) return fail(IE_ERR_INVALID, "queries contain NaN or infinite values");
+  }
+  std::lock_guard<std::mutex> lk(h->mu);
+  CK(cudaSetDevice(h->device));
+  cudaStream_t s = (stream || dev) ? static_cast<cudaStream_t>(stream) : h->own_stream;
+  if (h->has_done && s != h->last_stream) CK(cudaStreamWaitEvent(s, h->done_ev, 0));
+  const int grid = ie::knn_search_grid(h->n_pad, h->num_sms);
+  const int chunk = std::min(m, kKnnQueryChunk);
+  const int chunk_pad = static_cast<int>(round_up(chunk, 128));
+  CK(h->cand_s.reserve(static_cast<size_t>(chunk) * grid * k * sizeof(float)));
+  CK(h->cand_i.reserve(static_cast<size_t>(chunk) * grid * k * sizeof(int)));
+  if (!self) {
+    CK(h->qa.reserve(static_cast<size_t>(chunk_pad) * 2 * h->k_pad * sizeof(__nv_bfloat16), true));
+    CK(h->qomc.reserve(static_cast<size_t>(chunk) * sizeof(double)));
+    if (!dev) CK(h->qf.reserve(static_cast<size_t>(chunk) * d * sizeof(float)));
+  }
+  if (!dev) {
+    CK(h->dist.reserve(static_cast<size_t>(chunk) * k * sizeof(float)));
+    CK(h->ids.reserve(static_cast<size_t>(chunk) * k * sizeof(int64_t)));
+  }
+  CK(cudaMemsetAsync(h->err.p, 0, sizeof(unsigned), s));
+  for (long long q0 = 0; q0 < m; q0 += chunk) {
+    const int rows = static_cast<int>(std::min<long long>(chunk, m - q0));
+    ie::KnnSearchArgs a{};
+    a.index = h->index.as<__nv_bfloat16>();
+    a.bias = h->bias.as<float>();
+    a.n_valid = static_cast<int>(h->n);
+    a.n_pad = h->n_pad;
+    a.k_pad = h->k_pad;
+    a.m = rows;
+    a.k = k;
+    a.cand_s = h->cand_s.as<float>();
+    a.cand_i = h->cand_i.as<int>();
+    a.num_sms = h->num_sms;
+    a.abort_flag = h->err.as<unsigned>();
+    if (self) {
+      // the stored residuals of rows [row0 + q0, +rows) are the query operand: no prep
+      a.a = h->index.as<__nv_bfloat16>();
+      a.a_rows = h->n_pad;
+      a.a_row0 = static_cast<int>(row0 + q0);
+      a.self0 = row0 + q0;
+      a.omc = h->omc.as<double>() + row0 + q0;
+    } else {
+      const float* x = queries + q0 * d;
+      if (!dev) {
+        CK(cudaMemcpyAsync(h->qf.p, x, static_cast<size_t>(rows) * d * sizeof(float), cudaMemcpyHostToDevice, s));
+        x = h->qf.as<float>();
+      }
+      CK(ie::launch_knn_prep_rows(x, d, d, rows, h->mean.as<double>(), h->k_pad, h->qa.as<__nv_bfloat16>(), nullptr,
+                                  h->qomc.as<double>(), s));
+      a.a = h->qa.as<__nv_bfloat16>();
+      a.a_rows = chunk_pad;
+      a.a_row0 = 0;
+      a.self0 = -1;
+      a.omc = h->qomc.as<double>();
+    }
+    a.dist = dev ? distances + q0 * k : h->dist.as<float>();
+    a.ids = dev ? ids + q0 * k : h->ids.as<int64_t>();
+    CK(ie::launch_knn_search(a, s));
+    if (!dev) {
+      CK(cudaMemcpyAsync(distances + q0 * k, h->dist.p, static_cast<size_t>(rows) * k * sizeof(float),
+                         cudaMemcpyDeviceToHost, s));
+      CK(cudaMemcpyAsync(ids + q0 * k, h->ids.p, static_cast<size_t>(rows) * k * sizeof(int64_t), cudaMemcpyDeviceToHost,
+                         s));
+      CK(cudaStreamSynchronize(s));  // qf and the output staging are reused by the next chunk
+    }
+  }
+  CK(cudaEventRecord(h->done_ev, s));
+  h->last_stream = s;
+  h->has_done = true;
+  if (!dev) {
+    unsigned aborted = 0;
+    CK(cudaMemcpy(&aborted, h->err.p, sizeof(unsigned), cudaMemcpyDeviceToHost));
+    if (aborted) return fail(IE_ERR_CUDA, "a device-side wait of the search kernel exceeded its limit and was drained");
+  }
+  return IE_OK;
+}
+
+void ie_knn_destroy(ie_knn* h) {
+  if (h == nullptr) return;
+  cudaSetDevice(h->device);
+  cudaDeviceSynchronize();
+  delete h;
 }
 
 }  // extern "C"

@@ -125,4 +125,42 @@ constexpr int kPrMaxSamples = 16384;
 cudaError_t launch_pr_thresholds(const float* scores, const uint8_t* truth, int n, int n_labels, double p_thr,
                                  double r_thr, float* out_thr, double* out_prec, double* out_rec, cudaStream_t stream);
 
+// ---- exact cosine k-nearest-neighbour search (knn.cu) ---------------------------------------------------------------
+// Index prep: inv[r] = 1 / |x_r| (f64, 0 for a zero row); partial column sums of x * inv over blocks of 512 rows (rows
+// of this call land in partial blocks [blk0, blk0 + knn_colsum_blocks(rows))); mu = sum of the blocks in order / n.
+long long knn_colsum_blocks(long long rows);
+cudaError_t launch_knn_inv_norm(const float* x, long long ldx, int d, int rows, double* inv, cudaStream_t stream);
+cudaError_t launch_knn_colsum(const float* x, long long ldx, int d, int rows, const double* inv, double* partial,
+                              long long blk0, cudaStream_t stream);
+cudaError_t launch_knn_mean(const double* partial, long long nblk, int d, int k_pad, long long n, double* mu,
+                            cudaStream_t stream);
+// rows [rows, d] f32 -> out [rows, 2*k_pad] bf16 = [hi | lo] of f32(x/|x| - mu); bias[r] = f32(mu . r) (nullptr: not
+// written; queries), omc[r] = 1 - (x/|x|) . mu; all dot products in f64
+cudaError_t launch_knn_prep_rows(const float* x, long long ldx, int d, int rows, const double* mu, int k_pad,
+                                 __nv_bfloat16* out, float* bias, double* omc, cudaStream_t stream);
+// *flag = 1 if any of x[rows, d] (row pitch ldx) is NaN or infinite
+cudaError_t launch_knn_check_finite(const float* x, long long ldx, int d, long long rows, unsigned* flag,
+                                    cudaStream_t stream);
+constexpr int kKnnMaxK = 32;
+struct KnnSearchArgs {
+  const __nv_bfloat16* a;      // query operand [a_rows, 2*k_pad] (split-bf16 residuals); rows a_row0 .. a_row0 + m
+  long long a_rows;            // rows of the A tensor (reads past it are zero-filled by the TMA unit)
+  int a_row0;
+  const __nv_bfloat16* index;  // [n_pad, 2*k_pad]
+  const float* bias;           // [n_pad] b_x
+  int n_valid, n_pad, k_pad;   // n_pad % 256 == 0, k_pad % 64 == 0
+  long long self0;             // >= 0: query i is index row self0 + i and skips itself; -1: external queries
+  int m, k;                    // queries of this launch, neighbours per query (1..kKnnMaxK)
+  const double* omc;           // [m] 1 - c_q
+  float* cand_s;               // workspace [m, knn_search_grid(), k]
+  int* cand_i;
+  float* dist;                 // [m, k]
+  int64_t* ids;                // [m, k]
+  int num_sms;
+  unsigned* abort_flag;
+  long long spin_limit;
+};
+int knn_search_grid(int n_pad, int num_sms);
+cudaError_t launch_knn_search(const KnnSearchArgs& a, cudaStream_t stream);
+
 }  // namespace ie

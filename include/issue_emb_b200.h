@@ -154,6 +154,28 @@ int ie_pr_thresholds(const float* scores, const uint8_t* truth, int32_t n, int32
                      double recall_threshold, float* thresholds, double* precisions, double* recalls, int32_t device,
                      int32_t flags, void* stream);
 
+/* Similar-issue search: exact cosine k-nearest neighbours over an index of issue embeddings.  Replaces the host-side
+ * brute-force searches of the reference: the one-shot labeler of
+ * Issue_Embeddings/notebooks/scratch/Kubeflow-FewShotLearning.ipynb (cell 46, oneshotlabeler.query: CosineSimilarity
+ * against every labelled issue, then argsort(descending=True)) and KNeighborsClassifier(n_neighbors=2,
+ * weights='distance', metric='cosine') of cell 77 of the same notebook; the duplicate issues noted at
+ * Get-GitHub-Issues.ipynb:361 and 01_AcquireData.ipynb:48 are what a self-join finds.  The reference's README lists
+ * duplicate detection and reviewer recommendation as uses of the embedding; both are this search.
+ *
+ * Create: vectors [n, d] f32 (host, or device on `device` with IE_FLAG_DEVICE_PTRS, read on `stream`), 1 <= d <= 4096,
+ * all finite.  Synchronous.  The index keeps 4 * round_up(d, 64) bytes per row (split-bf16 residuals), plus 12 B. */
+typedef struct ie_knn ie_knn;
+int ie_knn_create(const float* vectors, int64_t n, int32_t d, int32_t device, int32_t flags, void* stream, ie_knn** out);
+/* Search, as sklearn NearestNeighbors(metric='cosine', algorithm='brute').kneighbors:
+ *   queries [m, d] f32 -> distances [m, k] f32 (1 - cos, ascending; ties: smaller id first), ids [m, k] int64.
+ *   queries == NULL: the queries are index rows [row0, row0 + m), each excluding itself (kneighbors(X=None)).
+ * 1 <= k <= 32 and k <= n (n - 1 for self-queries).  Zero vectors have cosine 0 with everything (distance 1).
+ * Host pointers: synchronous, non-finite queries are rejected.  IE_FLAG_DEVICE_PTRS: queries / distances / ids are
+ * device pointers and the call is asynchronous on `stream`. */
+int ie_knn_search(ie_knn* h, const float* queries, int64_t row0, int32_t m, int32_t k, float* distances, int64_t* ids,
+                  int32_t flags, void* stream);
+void ie_knn_destroy(ie_knn* h);
+
 /* Debug / test hook: D[M,N] = A[M,K] * B[N,K]^T (+bias) through the same tcgen05 GEMM the encoder uses.
  * a [M,K], b [N,K], bias [N] or NULL: host f32 (rounded to bf16 on the device); d [M,N] host f32. */
 int ie_debug_gemm(const float* a, const float* b, const float* bias, int32_t M, int32_t N, int32_t K, int32_t act,
